@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — schedule prefixes/sec on the BASELINE.json north-star workload, plus the secondary configs.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--no-secondary]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--no-secondary] [--dump-outputs DIR]
 
 Headline (BASELINE.json configs[1]): 5-actor Raft model (seeded double-vote bug), RandomScheduler/FullyRandom fuzz,
 maxMessages=50, invariant every 5 deliveries, 10^7 prefixes per step per GPU (weak scaling: rank r, step s explores
@@ -17,6 +17,10 @@ its own seed range).  One "step" = one pass of the hot path over one batch of pr
   secondary    : configs[2] (one DPORwHeuristics search as a frontier, with the in-library NCCL steal round at N > 1),
                  configs[3] (DDMin / STSSched replays over a 2000-event trace), configs[4] (bcast32 + state-hash
                  dedup) — measured after, and outside, the headline's timed region (tools/secondary.py)
+
+`--dump-outputs DIR` writes what the timed path computed in its last step on rank 0 (see dump_outputs) as
+DIR/<name>.npy, so that two builds can be compared output for output: the inputs depend on the arguments alone.
+The benchmark itself writes nothing into the tree; an oracle library it has to rebuild goes to a temporary directory.
 
 `--impl reference` times the CPU oracle alone on the SAME batch definition (the reference itself needs a JVM + sbt +
 Akka + the akka-raft application, none of which exist here).
@@ -137,14 +141,37 @@ def k1_profile(k1_id):
     return p, None
 
 
+DUMP_RECORDS = 1 << 18     # 11 float64 arrays of this length: 23 MB, well inside 64 MB
+
+
+def dump_outputs(out_dir, n, take, violations, deliveries):
+    """Write the last timed step's output as a caller of the fuzz path receives it: every field of the result records
+    of a fixed, seeded sample of DUMP_RECORDS records (all records when the batch is smaller; `take(idx)` returns them
+    as RESULT_DTYPE), 64-bit hashes split into exact 32-bit halves, and the step's violation / delivery counts."""
+    import numpy as np
+    from demi_b200 import _native as N
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.sort(np.random.default_rng(0).choice(n, DUMP_RECORDS, replace=False)) if n > DUMP_RECORDS else np.arange(n)
+    rec = take(idx)
+    arrays = {"record_index": idx, "counts": np.array([violations, deliveries])}
+    for f in N.RESULT_DTYPE.names:
+        v = rec[f].astype(np.uint64)
+        if N.RESULT_DTYPE[f].itemsize == 8:
+            arrays[f + "_lo"], arrays[f + "_hi"] = v & np.uint64(0xFFFFFFFF), v >> np.uint64(32)
+        else:
+            arrays[f] = v
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def run_reference(args):
     """CPU arm: the oracle on all host cores, the same batch definition as the GPU arm (same_config)."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return 0
-    from demi_b200 import build, events
-    build.build_oracle()
+    from demi_b200 import events
     from oracle import binding as O
+    O.lib(private=True)
     ext = events.pack_externals(events.raft5_program())
     cores = host_cores()
     n = args.prefixes
@@ -152,9 +179,12 @@ def run_reference(args):
         O.fuzz_batch(MODEL_RAFT5, ext, 1 + w * 100_000, 100_000, MAX_MESSAGES, INTERVAL, model_flags=MODEL_FLAGS, threads=cores)
     t0 = time.perf_counter()
     for s in range(args.steps):
-        O.fuzz_batch(MODEL_RAFT5, ext, 1 + (args.warmup + s) * n, n, MAX_MESSAGES, INTERVAL,
-                     model_flags=MODEL_FLAGS, threads=cores)
+        out = O.fuzz_batch(MODEL_RAFT5, ext, 1 + (args.warmup + s) * n, n, MAX_MESSAGES, INTERVAL,
+                           model_flags=MODEL_FLAGS, threads=cores)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, n, lambda idx: out[idx], int((out["violation"] != 0).sum()),
+                     int(out["steps"].sum(dtype="u8")))
     value = n * args.steps / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": "prefixes/s", "n_gpus": args.gpus,
@@ -180,7 +210,10 @@ def main():
     ap.add_argument("--prefixes", type=int, default=PREFIXES_PER_STEP)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.prefixes < 1:
+        ap.error("--steps and --prefixes must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -200,9 +233,6 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
 
     import demi_b200 as D
-    from demi_b200 import build
-    if not os.path.exists(build.LIB):
-        build.build_engine()
     n = args.prefixes
     W, K = max(args.warmup, 0), args.steps
     eng = D.Engine(D.SchedulerConfig(MODEL_RAFT5, model_flags=MODEL_FLAGS, device=local_rank))
@@ -241,6 +271,11 @@ def main():
     total_ms = evs[0].elapsed_time(evs[K])
     kernel_ms = [evs[i].elapsed_time(evs[i + 1]) for i in range(K)]
     nv, ss = eng.fuzz_summary_dev(stream.cuda_stream)   # counters of the last step
+    if args.dump_outputs and rank == 0:
+        records = results_dev.view(n, RESULT_BYTES)
+        dump_outputs(args.dump_outputs, n,
+                     lambda idx: records[torch.from_numpy(idx).to(dev)].cpu().numpy().reshape(-1).view(D._native.RESULT_DTYPE),
+                     nv, ss)
     t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
     cnt = torch.tensor([float(nv), float(ss)], dtype=torch.float64, device=dev)
     if world > 1:
@@ -311,7 +346,7 @@ def main():
         line["cpu_baseline"] = None                 # timed at N=1 only (rank 0)
         if not args.no_cpu_baseline and world == 1:
             from oracle import binding as O
-            build.build_oracle()
+            O.lib(private=True)
             cores = host_cores()
             ncpu = 125_000 * cores
             O.fuzz_batch(MODEL_RAFT5, ext, 1, 50_000, MAX_MESSAGES, INTERVAL, model_flags=MODEL_FLAGS, threads=cores)

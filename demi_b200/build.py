@@ -96,13 +96,20 @@ def _cpu_stamp():
 ORACLE_STAMP = os.path.join(ORACLE_DIR, ".build_cpu")
 
 
-def build_oracle(force=False):
+def build_oracle(force=False, private=False):
+    """Return the path of an oracle library built for this CPU.  private=True leaves the tree untouched: a missing
+    or stale in-tree library is then built in a new temporary directory (bench.py may run from a read-only tree)."""
     srcs = _sources(ORACLE_DIR, (".c", ".h")) + _sources(os.path.join(ROOT, "include"), (".h",))
     srcs.append(os.path.join(ORACLE_DIR, "Makefile"))
     stamp = _cpu_stamp()
     same_cpu = os.path.exists(ORACLE_STAMP) and open(ORACLE_STAMP).read().strip() == stamp
     if not force and same_cpu and _newer(ORACLE_LIB, srcs):
         return ORACLE_LIB
+    if private:
+        import tempfile
+        out = os.path.join(tempfile.mkdtemp(prefix="demi_oracle_"), "liboracle.so")
+        subprocess.check_call(["make", "-B", "-C", ORACLE_DIR, "OUT=" + out, out], stdout=sys.stderr)
+        return out
     # make's chatter goes to stderr: bench.py prints exactly one JSON line on stdout
     subprocess.check_call(["make", "-B", "-C", ORACLE_DIR, "liboracle.so"], stdout=sys.stderr)
     with open(ORACLE_STAMP, "w") as f:

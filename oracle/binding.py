@@ -33,15 +33,20 @@ class FuzzParams(C.Structure):
 _lib = None
 
 
-def lib():
+def lib(private=False):
+    """Load the oracle once.  private=True: never write into the tree (see build.build_oracle); a library built
+    elsewhere is removed as soon as it is loaded."""
     global _lib
     if _lib is None:
         # -march=native build: (re)built on the machine that runs it (demi_b200/build.py keeps a CPU stamp)
         import sys
         sys.path.insert(0, os.path.dirname(_HERE))
         from demi_b200 import build
-        build.build_oracle()
-        _lib = C.CDLL(LIB_PATH)
+        path = build.build_oracle(private=private)
+        _lib = C.CDLL(path)
+        if path != LIB_PATH:
+            import shutil
+            shutil.rmtree(os.path.dirname(path))
     return _lib
 
 

@@ -1,5 +1,6 @@
 // C++ host mirror (include/demi_b200.hpp) end to end.  With a CUDA device: fuzz -> DDMin -> verify ->
 // internal minimization -> strict replay -> DPOR.  Without: the no-CPU-fallback contract.
+// argv[1]: a directory the experiment round trip may create (the test passes a private temporary one).
 #include <cstdio>
 #include <cstdlib>
 #include "demi_b200.hpp"
@@ -8,7 +9,7 @@ using namespace demi;
 
 #define CHECK(c) do { if (!(c)) { std::printf("CHECK failed: %s (line %d)\n", #c, __LINE__); return 1; } } while (0)
 
-int main() {
+int main(int argc, char** argv) {
   SchedulerConfig cfg;
   cfg.model = DEMI_MODEL_RAFT5;
   cfg.model_flags = 1;
@@ -124,7 +125,8 @@ int main() {
     CHECK(same && differs);
     Experiment x; x.model = cfg.model; x.model_flags = cfg.model_flags; x.violation = fp; x.externals = prog; x.trace = trace;
     x.dep_parent = sched.depGraph; x.mcs_mask = mask_of(prog, mcs);
-    const std::string dir = "/tmp/demi_b200_cpp_experiment";
+    CHECK(argc > 1);
+    const std::string dir = argv[1];
     x.save(dir);
     Experiment y = Experiment::load(dir);
     CHECK(y.model == x.model && y.violation == fp && y.externals.size() == prog.size() && y.trace.size() == trace.size());

@@ -25,7 +25,7 @@ def test_cpp_mirror_builds_and_refuses_to_run_without_a_gpu(native):
 
 
 @pytest.mark.gpu
-def test_cpp_mirror_pipeline_on_gpu(native):
+def test_cpp_mirror_pipeline_on_gpu(native, tmp_path):
     build(native)           # always: a binary left by an earlier run may predate the header
-    out = subprocess.run([EXE], capture_output=True, text=True, timeout=600)
+    out = subprocess.run([EXE, str(tmp_path / "experiment")], capture_output=True, text=True, timeout=600)
     assert out.returncode == 0 and out.stdout.strip().endswith("OK"), out.stdout + out.stderr
