@@ -23,10 +23,18 @@
 // prefix that completes here has, by construction, the same result as in the
 // general engine.
 #pragma once
+#include <type_traits>
 #include "machine.cuh"
 #include "models/models.cuh"
 
 namespace demi {
+
+// Does the model split receive() into lane_decide() + plan_item() (`static constexpr bool LANE_PLAN = true`, see
+// Raft5)?  Then the lane engine produces receive()'s sends itself (LaneMachine::plan_sends_produced).
+template <class M, class = void>
+struct lane_plan_model { static constexpr bool value = false; };
+template <class M>
+struct lane_plan_model<M, std::void_t<decltype(M::LANE_PLAN)>> { static constexpr bool value = M::LANE_PLAN; };
 
 #ifndef DEMI_K1_PEND_HINT
 #define DEMI_K1_PEND_HINT 1      // pending array accessed with an L2 evict_last policy
@@ -151,6 +159,9 @@ struct LaneMachine {
   static constexpr bool DIRECT = DEMI_K1_DIRECT_OUTBOX && MODEL::LANE_SENDS_DISTINCT;
   static constexpr int OBW = DIRECT ? 0 : OB * 3;
   static constexpr int WORDS = N * SW + OBW + N;       // states + outbox + partition rows
+  // receive()'s sends produced from the model's plan (recording runs keep receive()'s own send loop, whose
+  // record_event() also writes the EventTrace)
+  static constexpr bool PLAN = DIRECT && lane_plan_model<MODEL>::value && !REC;
 
   uint32_t* smw;             // &smem[tid]; word w at smw[w*BD]
   uint4* pend;               // entry i at pend[i*32]
@@ -444,7 +455,10 @@ struct LaneMachine {
     int slot = MODEL::timer_slot(dst, type, pick.y, pick.z);
     if (slot >= 0 && ((registry >> slot) & 1u)) enqueue_timer((uint32_t)slot);     // re-arm :1008-1016
     if (status) return 0;
-    if constexpr (DIRECT) {
+    if constexpr (PLAN) {
+      dispatch_plan(dst, src, type, pick.y, pick.z);
+      return 0;
+    } else if constexpr (DIRECT) {
       LaneDirectOutbox<LaneMachine> direct{this, dst};
       MODEL::receive(direct, dst, actor(dst), src, type, pick.y, pick.z, A->model_flags);
       return 0;
@@ -473,6 +487,48 @@ struct LaneMachine {
         }
     }
     return ob.n;
+  }
+
+  // receive() of a PLAN model, in its order: state update and cancel, then the sends, then the schedule
+  template <class MM = MODEL>
+  __device__ __forceinline__ void dispatch_plan(uint32_t self, uint32_t src, uint32_t type, uint32_t p0, uint32_t p1) {
+    LaneDirectOutbox<LaneMachine> direct{this, self};
+    const typename MM::Plan p = MODEL::lane_decide(direct, self, actor(self), src, type, p0, p1, A->model_flags);
+    plan_sends_produced<MM>(p, self, src);
+    if (p.sched) schedule_timer(OP_SCHED_REPEAT, self, p.sched, 0, 0);
+  }
+  // actor_send_produced() for each send of plan `p`, in plan order.  While nobody is isolated or partitioned and the
+  // node and pending capacities hold all of the sends, every send is inserted and none defers, so the ids, trace
+  // positions and pending slots of send k are simply the next ones plus k, and the counters advance once for the
+  // whole plan.  (No send of a plan is a timer key, so the cancelled-timer rule never drops one.)  Otherwise each
+  // send goes through actor_send_produced().
+  template <class MM = MODEL>
+  __device__ __forceinline__ void plan_sends_produced(const typename MM::Plan& p, uint32_t self, uint32_t src) {
+    const uint32_t n = MODEL::plan_sends(p);
+    if (status || n == 0) return;
+    LaneState s = actor(self);
+    if ((inaccessible | killed) || A->has_partitions || n_nodes + n > A->node_cap ||
+        n_pending + n > A->pending_cap || n_pending + n > (uint32_t)LPCAP) {
+#pragma unroll 1
+      for (uint32_t k = 0; k < n; k++) {
+        uint32_t dst, type, q0, q1;
+        MODEL::plan_item(p, self, src, k, s, s, dst, type, q0, q1);
+        actor_send_produced(self, dst, type, q0, q1);
+      }
+      return;
+    }
+#pragma unroll 1
+    for (uint32_t k = 0; k < n; k++) {
+      uint32_t dst, type, q0, q1;
+      MODEL::plan_item(p, self, src, k, s, s, dst, type, q0, q1);
+      const uint32_t w3 = (n_uniq + 1u + k) | ((n_nodes + k) << 16);
+      st_l2_hint(pend + (n_pending + k) * 32, make_uint4(make_hdr(self, dst, type, 0), q0, q1, w3), pol);
+      thash += demi_event_term(DEMI_EV_MSG_SEND | (self << 8) | (dst << 16) | (type << 24), q0, q1, w3,
+                               n_events + k, parent_event);
+    }
+    n_uniq += n; n_nodes += n; n_events += n;
+    n_pending += n;
+    if (n_pending > max_pending) max_pending = n_pending;       // nothing is removed between the inserts
   }
 
   __device__ __forceinline__ void reset(int64_t seed) {

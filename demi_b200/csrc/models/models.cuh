@@ -138,22 +138,64 @@ struct Raft5 {
   __device__ static __forceinline__ void receive(O& out, uint32_t self, S s, uint32_t src,
                                                  uint32_t type, uint32_t p0, uint32_t p1, uint32_t flags) {
     Scalars<S> c(s);
-    receive_body(out, self, s, c, src, type, p0, p1, flags);
+    const Plan p = decide(out, self, s, c, src, type, p0, p1, flags);
+#pragma unroll 1
+    for (uint32_t k = 0; k < plan_sends(p); k++) {
+      uint32_t dst, qt, q0, q1;
+      plan_item(p, self, src, k, s, c, dst, qt, q0, q1);
+      out.send(dst, qt, q0, q1);
+    }
+    if (p.sched) out.schedule_repeating(p.sched, 0, 0);
     c.flush(s);
   }
   // Every handler emits its operations in the order: cancel (step_down), then its sends, then schedule.  The sends
-  // are either one reply to the sender or one message per peer, so the handlers only DESCRIBE their operations and
-  // these leave through ONE cancel, ONE send and ONE schedule site after the switch: engines that apply an operation
-  // as it is issued (the lane engine) then carry one copy of that code instead of one per handler, and the threads of
-  // a warp that handle different message types meet again at those sites.
+  // are either one reply to the sender or one message per peer, so the handlers only DESCRIBE their operations (a
+  // Plan, returned by decide() after the cancel) and these leave through ONE send and ONE schedule site after the
+  // switch: engines that apply an operation as it is issued then carry one copy of that code instead of one per
+  // handler, and the threads of a warp that handle different message types meet again at those sites.
+  //
+  // The lane engine (LANE_PLAN) calls lane_decide() and produces the sends itself from plan_item(): send k of a plan,
+  // computed from the sender's state after decide().  No type a plan sends is a timer key (timer_slot < 0), so the
+  // cancelled-timer rule never drops one of these sends.
+  static constexpr bool LANE_PLAN = true;
   enum { PLAN_NONE = 0, PLAN_REPLY = 1, PLAN_REQUEST_VOTES = 2, PLAN_APPEND_ALL = 3 };
+  struct Plan { uint32_t kind, type, p0, sched; };
+  __device__ static __forceinline__ uint32_t plan_sends(const Plan& p) {
+    return p.kind == PLAN_NONE ? 0u : p.kind == PLAN_REPLY ? 1u : 4u;
+  }
+  // send k of plan p: a reply goes to the sender, the others to every peer in ascending order, skipping `self`
+  template <class S, class C>
+  __device__ static __forceinline__ void plan_item(const Plan& p, uint32_t self, uint32_t src, uint32_t k, S& s, C& c,
+                                                   uint32_t& dst, uint32_t& type, uint32_t& q0, uint32_t& q1) {
+    dst = p.kind == PLAN_REPLY ? src : k + (k >= self ? 1u : 0u);
+    type = p.kind == PLAN_REPLY ? p.type : (uint32_t)REQUEST_VOTE;
+    q0 = p.p0; q1 = 0;
+    if (p.kind == PLAN_APPEND_ALL) {
+      const uint32_t prev = s[NEXT + dst];
+      const uint32_t pt = prev ? s[LOGTERM + prev - 1] : 0u;
+      const uint32_t has = prev < c[LOGLEN] ? 1u : 0u;
+      const uint32_t et = has ? s[LOGTERM + prev] : 0u, ev = has ? s[LOGVAL + prev] : 0u;
+      type = APPEND_ENTRIES;
+      q0 = (uint32_t)c[TERM] | (prev << 8) | (pt << 16) | ((uint32_t)c[COMMIT] << 24);
+      q1 = has | (et << 8) | (ev << 16);
+    }
+  }
+  // receive() up to and including its cancel; the state is written back, so plan_item() may read it from `s` alone
+  template <class S, class O>
+  __device__ static __forceinline__ Plan lane_decide(O& out, uint32_t self, S s, uint32_t src,
+                                                     uint32_t type, uint32_t p0, uint32_t p1, uint32_t flags) {
+    Scalars<S> c(s);
+    const Plan p = decide(out, self, s, c, src, type, p0, p1, flags);
+    c.flush(s);
+    return p;
+  }
   template <class S, class C, class O>
-  __device__ static __forceinline__ void receive_body(O& out, uint32_t self, S& s, C& c, uint32_t src,
-                                                      uint32_t type, uint32_t p0, uint32_t p1, uint32_t flags) {
+  __device__ static __forceinline__ Plan decide(O& out, uint32_t self, S& s, C& c, uint32_t src,
+                                                uint32_t type, uint32_t p0, uint32_t p1, uint32_t flags) {
     const uint32_t last_idx = c[LOGLEN];
     const uint32_t last_term = last_idx ? s[LOGTERM + last_idx - 1] : 0u;
     const uint32_t t = p0 & 0xFF;
-    if (type != BOOT && type != CLIENT_CMD && c[ROLE] == INIT) return;
+    if (type != BOOT && type != CLIENT_CMD && c[ROLE] == INIT) return Plan{PLAN_NONE, 0, 0, 0};
     uint32_t plan = PLAN_NONE, plan_type = 0, plan_p0 = 0, sched = 0;
     bool cancel_heartbeat = false;
     switch (type) {
@@ -255,24 +297,7 @@ struct Raft5 {
       default: break;
     }
     if (cancel_heartbeat) out.cancel_timer(HEARTBEAT_TICK, 0, 0);
-    if (plan != PLAN_NONE) {
-#pragma unroll 1
-      for (uint32_t j = (plan == PLAN_REPLY ? src : 0u), end = (plan == PLAN_REPLY ? src + 1u : 5u); j < end; j++) {
-        if (plan != PLAN_REPLY && j == self) continue;
-        uint32_t q0 = plan_p0, q1 = 0, qt = plan == PLAN_REPLY ? plan_type : (uint32_t)REQUEST_VOTE;
-        if (plan == PLAN_APPEND_ALL) {
-          const uint32_t prev = s[NEXT + j];
-          const uint32_t pt = prev ? s[LOGTERM + prev - 1] : 0u;
-          const uint32_t has = prev < c[LOGLEN] ? 1u : 0u;
-          const uint32_t et = has ? s[LOGTERM + prev] : 0u, ev = has ? s[LOGVAL + prev] : 0u;
-          qt = APPEND_ENTRIES;
-          q0 = (uint32_t)c[TERM] | (prev << 8) | (pt << 16) | ((uint32_t)c[COMMIT] << 24);
-          q1 = has | (et << 8) | (ev << 16);
-        }
-        out.send(j, qt, q0, q1);
-      }
-    }
-    if (sched) out.schedule_repeating(sched, 0, 0);
+    return Plan{plan, plan_type, plan_p0, sched};
   }
 
   // lanes 0..9 each own one unordered pair (i<j).  code 1: two leaders in one
