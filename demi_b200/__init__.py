@@ -6,4 +6,4 @@ from .events import (Start, Kill, HardKill, Send, WaitQuiescence, Partition, UnP
 from .schedulers import (DemiError, SchedulerConfig, Engine, RandomScheduler, STSScheduler, ReplayScheduler,  # noqa: F401
                          DDMin, MinimizationStats, DPORwHeuristics, STSSchedMinimizer, LeftToRightOneAtATime, SrcDstFIFORemoval,
                          ProvenanceTracker, ResumableDPOR, IncrementalDDMin, ArvindDistanceOrdering,
-                         DefaultBacktrackOrdering, mask_of, events_of)
+                         DefaultBacktrackOrdering, mask_of, events_of, program_of, random_ddmin)

@@ -106,6 +106,7 @@ EXPORTS = [
     "demi_dpor_frontier", "demi_dpor_frontier_multi", "demi_comm_unique_id", "demi_comm_init", "demi_comm_rank",
     "demi_create_multi", "demi_conjoin_atoms", "demi_fuzzer_generate", "demi_experiment_save", "demi_experiment_load",
     "demi_load_model", "demi_actor_index", "demi_actor_name", "demi_set_user_filter",
+    "demi_fuzz_subseq_batch", "demi_random_ddmin",
 ]
 FILTER_RULE_DTYPE = np.dtype([("src_mask", "<u4"), ("dst_mask", "<u4"), ("type_mask", "<u4"), ("flags", "<u4")])
 FRULE_DEADLETTERS = 1
@@ -240,6 +241,11 @@ def lib():
     L.demi_experiment_load.argtypes = [C.c_char_p, C.POINTER(Experiment)]
     L.demi_conjoin_atoms.restype = C.c_int32
     L.demi_conjoin_atoms.argtypes = [vp, C.c_uint32, C.c_uint32]
+    L.demi_fuzz_subseq_batch.restype = C.c_int32
+    L.demi_fuzz_subseq_batch.argtypes = [vp, C.POINTER(FuzzParams), vp, C.c_uint32, C.c_uint32, vp, vp]
+    L.demi_random_ddmin.restype = C.c_int32
+    L.demi_random_ddmin.argtypes = [vp, C.POINTER(FuzzParams), vp, C.c_uint32, C.c_int32, vp, C.c_uint32, vp, vp,
+                                    C.c_uint32, C.POINTER(DDMinOut), C.POINTER(C.c_int64)]
     L.demi_stats.restype = C.c_int32
     L.demi_stats.argtypes = [vp, C.POINTER(Perf)]
     _lib = L

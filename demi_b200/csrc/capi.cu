@@ -12,6 +12,7 @@
 #include "fuzz_kernel.cuh"
 #include "provenance_kernel.cuh"
 #include "lane_kernel.cuh"
+#include "subseq_kernel.cuh"
 #include "models/model_ir.cuh"
 
 using namespace demi;
@@ -23,15 +24,19 @@ thread_local std::string g_create_error;
 // ------------------------------------------------------------ kernel table
 constexpr int WARPS = 4;
 typedef void (*kernel_fn)(const KernelArgs);
+typedef void (*subseq_fn)(const SubseqArgs);
 struct Variant {
   int model; uint32_t pcap, tcap; bool pend_global, record;
   kernel_fn fn; size_t smem_per_warp;
+  subseq_fn sub;             // the same machine in subsequence mode (non-recording variants)
 };
 template <class MODEL, int PCAP, int TCAP, bool PG, bool REC>
 static Variant make_variant() {
   using M = Machine<MODEL, PCAP, TCAP, PG, REC>;
+  subseq_fn sub = nullptr;
+  if constexpr (!REC) sub = fuzz_subseq_kernel<MODEL, PCAP, TCAP, PG, WARPS>;
   return Variant{MODEL::ID, (uint32_t)PCAP, (uint32_t)TCAP, PG, REC,
-                 fuzz_kernel<MODEL, PCAP, TCAP, PG, REC, WARPS>, sizeof(typename M::Smem)};
+                 fuzz_kernel<MODEL, PCAP, TCAP, PG, REC, WARPS>, sizeof(typename M::Smem), sub};
 }
 static const std::vector<Variant>& variants() {
   static const std::vector<Variant> v = {
@@ -59,12 +64,12 @@ static const Variant* pick_variant(int model, uint32_t pcap, uint32_t tcap, bool
 }
 
 // lane-engine table
-struct LaneVariant { int model; int bd; uint32_t lpcap; kernel_fn fn; kernel_fn fn_rec; size_t smem_per_block; };
+struct LaneVariant { int model; int bd; uint32_t lpcap; kernel_fn fn; kernel_fn fn_rec; size_t smem_per_block; subseq_fn fn_sub; };
 template <class MODEL, int BD, int LPCAP>
 static LaneVariant make_lane_variant() {
   using M = LaneMachine<MODEL, BD, LPCAP>;
   return LaneVariant{MODEL::ID, BD, (uint32_t)LPCAP, fuzz_lane_kernel<MODEL, BD, LPCAP>, fuzz_lane_kernel<MODEL, BD, LPCAP, true>,
-                     (size_t)M::WORDS * BD * sizeof(uint32_t)};
+                     (size_t)M::WORDS * BD * sizeof(uint32_t), fuzz_lane_subseq_kernel<MODEL, BD, LPCAP>};
 }
 static const LaneVariant* pick_lane_variant(const demi_handle* h);
 
@@ -131,7 +136,7 @@ extern "C" void demi_destroy(demi_handle* h) {
   demi_replay_free(h);
   demi_frontier_free(h);
   demi_comm_free(h);
-  cudaFree(h->ir_blob_dev); cudaFree(h->trace_rec);
+  cudaFree(h->ir_blob_dev); cudaFree(h->trace_rec); cudaFree(h->subseq_buf);
   cudaFree(h->dedup.keys); cudaFree(h->dedup.vals); cudaFree(h->dedup.keep); cudaFree(h->dedup.counts);
   if (h->pinned) cudaFreeHost(h->pinned);
   if (h->ev0) cudaEventDestroy(h->ev0);
@@ -526,6 +531,168 @@ extern "C" int32_t demi_fuzz_trace(demi_handle* h, const demi_fuzz_params* p, in
   if (n_nodes) *n_nodes = counts[1];
   if (result) *result = r;
   if (r.status) return fail(h, DEMI_ERR_CAPACITY, "demi_fuzz_trace: prefix status %u", (unsigned)r.status);
+  return DEMI_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// Subsequence batches: RandomScheduler.test of many subsequences of the program in one launch (subseq_kernel.cuh)
+
+// program_of(mask) (include/demi_b200.h) as a mask: adjacent WaitQuiescence collapsed.  Returns n_eff (last selected
+// index + 1) and the number of Sends; 0 for an empty selection.
+static uint32_t subseq_effective(const std::vector<demi_ext_event>& ext, const uint64_t* m, uint64_t* eff, uint32_t* sends) {
+  uint32_t n_eff = 0, ns = 0; bool prev_wq = false;
+  for (uint32_t j = 0; j < (uint32_t)ext.size(); j++) {
+    if (!((m[j >> 6] >> (j & 63)) & 1ull)) continue;
+    const bool wq = ext[j].kind == DEMI_EXT_WAIT_QUIESCENCE;
+    if (wq && prev_wq) continue;
+    prev_wq = wq;
+    eff[j >> 6] |= 1ull << (j & 63);
+    if (ext[j].kind == DEMI_EXT_SEND) ns++;
+    n_eff = j + 1;
+  }
+  *sends = ns;
+  return n_eff;
+}
+
+extern "C" int32_t demi_fuzz_subseq_batch(demi_handle* h, const demi_fuzz_params* p, const uint64_t* masks, uint32_t n_tests,
+                                          uint32_t mask_words, uint32_t* first_hit, uint32_t* first_bad) {
+  if (!h) return DEMI_ERR_INVALID;
+  if (!p) return fail(h, DEMI_ERR_INVALID, "null params");
+  if (!n_tests) return DEMI_OK;
+  if (!masks || !first_hit || !first_bad) return fail(h, DEMI_ERR_INVALID, "demi_fuzz_subseq_batch: masks, first_hit and first_bad are required");
+  if (h->ext_host.empty()) return fail(h, DEMI_ERR_STATE, "demi_set_externals has not been called");
+  if (p->n_prefixes > 0xFFFFFFFFull) return fail(h, DEMI_ERR_INVALID, "n_prefixes > 2^32-1 per call");
+  { int32_t mrc = demi_need_model(h); if (mrc != DEMI_OK) return mrc; }
+  const uint32_t n_ext = (uint32_t)h->ext_host.size(), mw = mask_words, K = (uint32_t)p->n_prefixes;
+  if (!mw || (uint64_t)mw * 64 < n_ext) return fail(h, DEMI_ERR_INVALID, "demi_fuzz_subseq_batch: %u mask words cannot hold %u externals", mw, n_ext);
+  // the per-test side table: effective mask, n_eff, capacities of program_of(mask)
+  std::vector<uint64_t> eff((size_t)n_tests * mw, 0);
+  std::vector<uint32_t> n_eff(n_tests), sends(n_tests);
+  for (uint32_t t = 0; t < n_tests; t++) {
+    const uint64_t* m = masks + (size_t)t * mw;
+    for (uint32_t w = 0; w < mw; w++) {
+      const uint64_t valid = (uint64_t)w * 64 + 64 <= n_ext ? ~0ull : (uint64_t)w * 64 >= n_ext ? 0ull : ((1ull << (n_ext - w * 64)) - 1);
+      if (m[w] & ~valid) return fail(h, DEMI_ERR_INVALID, "demi_fuzz_subseq_batch: test %u selects an external beyond the %u of the program", t, n_ext);
+    }
+    n_eff[t] = subseq_effective(h->ext_host, m, &eff[(size_t)t * mw], &sends[t]);
+    if (!n_eff[t]) return fail(h, DEMI_ERR_INVALID, "demi_fuzz_subseq_batch: test %u selects no external", t);
+  }
+  if (K == 0) { std::fill(first_hit, first_hit + n_tests, 0u); std::fill(first_bad, first_bad + n_tests, 0u); return DEMI_OK; }
+  CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+  // the kernel variant and the scratch are those of the whole program: its capacities bound every subsequence's
+  const uint32_t per_chunk = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(n_tests, 0xFFFFFFFFull / K));
+  demi_fuzz_params q = *p;
+  q.n_prefixes = (uint64_t)per_chunk * K;
+  LaunchPlan plan;
+  int32_t rc = plan_launch(h, &q, false, &plan);
+  if (rc != DEMI_OK) return rc;
+  if (!plan.v->sub) return fail(h, DEMI_ERR_STATE, "demi_fuzz_subseq_batch: no subsequence kernel for the variant");
+  const LaneVariant* lv = pick_lane_variant(h);
+  std::vector<KernelArgs> ta(n_tests), tl(lv ? n_tests : 0);
+  for (uint32_t t = 0; t < n_tests; t++) {
+    KernelArgs a = plan.args;
+    a.n_ext = n_eff[t];
+    a.pending_cap = demi_pending_cap(demi_model_key(h), p->max_messages, sends[t]);
+    a.tosend_cap = demi_tosend_cap(sends[t]);
+    a.node_cap = demi_node_cap(a.pending_cap);
+    a.results = nullptr; a.sum_steps = nullptr; a.n_violations = nullptr;
+    ta[t] = a;
+    if (lv) {
+      a.ext_sends = h->ext_sends_dev;
+      a.has_partitions = h->has_partitions ? 1u : 0u;       // of the whole program: a fast-path flag only
+      if (h->lane_pending_cap) a.pending_cap = std::min(a.pending_cap, h->lane_pending_cap);
+      tl[t] = a;
+    }
+  }
+  // one device buffer: warp args | lane args | masks | first_hit | first_bad
+  auto al = [](size_t x) { return (x + 15) & ~(size_t)15; };
+  const size_t b_ta = al(ta.size() * sizeof(KernelArgs)), b_tl = al(tl.size() * sizeof(KernelArgs)),
+               b_m = al(eff.size() * sizeof(uint64_t)), b_v = al((size_t)n_tests * sizeof(uint32_t));
+  if ((rc = ensure(h, &h->subseq_buf, &h->subseq_buf_bytes, b_ta + b_tl + b_m + 2 * b_v)) != DEMI_OK) return rc;
+  unsigned char* d = (unsigned char*)h->subseq_buf;
+  KernelArgs* d_ta = (KernelArgs*)d; KernelArgs* d_tl = (KernelArgs*)(d + b_ta);
+  uint64_t* d_m = (uint64_t*)(d + b_ta + b_tl);
+  uint32_t* d_fh = (uint32_t*)(d + b_ta + b_tl + b_m); uint32_t* d_fb = (uint32_t*)(d + b_ta + b_tl + b_m + b_v);
+  std::vector<unsigned char> stage(b_ta + b_tl + b_m + 2 * b_v, 0);
+  memcpy(stage.data(), ta.data(), ta.size() * sizeof(KernelArgs));
+  if (lv) memcpy(stage.data() + b_ta, tl.data(), tl.size() * sizeof(KernelArgs));
+  memcpy(stage.data() + b_ta + b_tl, eff.data(), eff.size() * sizeof(uint64_t));
+  std::fill((uint32_t*)(stage.data() + b_ta + b_tl + b_m), (uint32_t*)(stage.data() + b_ta + b_tl + b_m) + n_tests, K);
+  std::fill((uint32_t*)(stage.data() + b_ta + b_tl + b_m + b_v), (uint32_t*)(stage.data() + b_ta + b_tl + b_m + b_v) + n_tests, K);
+  cudaStream_t s = h->stream;
+  CUDA_TRY(h, cudaMemcpyAsync(d, stage.data(), stage.size(), cudaMemcpyHostToDevice, s));
+  CUDA_TRY(h, cudaMemsetAsync(h->counters_dev, 0, 4 * sizeof(unsigned long long), s));
+  CUDA_TRY(h, cudaEventRecord(h->ev0, s));
+  h->perf.kernel_launches = 0;
+  if (h->cfg.model == DEMI_MODEL_IR) CUDA_TRY(h, ir_bind(h->ir_dev, s));
+  for (uint32_t t0 = 0; t0 < n_tests; t0 += per_chunk) {
+    const uint32_t nt = std::min(per_chunk, n_tests - t0);
+    const uint64_t items = (uint64_t)nt * K;
+    SubseqArgs sa{};
+    sa.targs = d_ta + t0; sa.targs_lane = lv ? d_tl + t0 : nullptr;
+    sa.masks = d_m + (size_t)t0 * mw; sa.mask_words = mw; sa.n_tests = nt;
+    sa.n_items = items; sa.seed_base = p->seed_base;
+    sa.first_hit = d_fh + t0; sa.first_bad = d_fb + t0;
+    sa.counters = h->counters_dev;
+    sa.node_scratch = h->node_scratch; sa.pend_scratch = h->pend_scratch; sa.fifo_scratch = plan.args.fifo_scratch;
+    sa.node_stride = plan.args.node_cap;
+    if (lv) {
+      // K1-lane runs every item it can prove exact; the rest go to the warp engine, as in demi_fuzz_batch
+      int bps = 0;
+      auto it = h->occupancy.find((const void*)lv->fn_sub);
+      if (it == h->occupancy.end()) {
+        CUDA_TRY(h, cudaFuncSetAttribute(lv->fn_sub, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lv->smem_per_block));
+        CUDA_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, lv->fn_sub, lv->bd, lv->smem_per_block));
+        h->occupancy[(const void*)lv->fn_sub] = bps;
+      } else bps = it->second;
+      if (bps < 1) return fail(h, DEMI_ERR_CAPACITY, "lane kernel does not fit on an SM");
+      const int lgrid = (int)std::max<uint64_t>(1, std::min<uint64_t>((items + lv->bd - 1) / lv->bd, (uint64_t)h->sm_count * bps));
+      const uint64_t lwarps = (uint64_t)lgrid * (lv->bd / 32);
+      if ((rc = ensure(h, (void**)&h->lane_pend, &h->lane_pend_bytes, lwarps * lv->lpcap * 32 * sizeof(uint4))) != DEMI_OK) return rc;
+      if ((rc = ensure(h, (void**)&h->ovf_list, &h->ovf_list_bytes, std::max<size_t>(items * sizeof(uint32_t), 64))) != DEMI_OK) return rc;
+      CUDA_TRY(h, cudaMemsetAsync(h->ovf_count, 0, sizeof(uint32_t), s));
+      sa.lane_pend = h->lane_pend; sa.ovf_list = h->ovf_list; sa.ovf_count = h->ovf_count;
+      lv->fn_sub<<<lgrid, lv->bd, lv->smem_per_block, s>>>(sa);
+      CUDA_TRY(h, cudaGetLastError());
+      h->perf.kernel_launches++;
+      sa.index_list = h->ovf_list; sa.index_count = h->ovf_count;
+      sa.ovf_list = nullptr; sa.ovf_count = nullptr;
+    }
+    {
+      auto it = h->occupancy.find((const void*)plan.v->sub);
+      if (it == h->occupancy.end()) {
+        int bps = 0;
+        CUDA_TRY(h, cudaFuncSetAttribute(plan.v->sub, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem));
+        CUDA_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, plan.v->sub, WARPS * 32, plan.smem));
+        if (bps < 1) return fail(h, DEMI_ERR_CAPACITY, "subsequence kernel does not fit on an SM (smem %zu)", plan.smem);
+        h->occupancy[(const void*)plan.v->sub] = bps;
+      }
+    }
+    // the warp grid (and the scratch behind it) was planned for per_chunk * K items
+    plan.v->sub<<<plan.grid, WARPS * 32, plan.smem, s>>>(sa);
+    CUDA_TRY(h, cudaGetLastError());
+    h->perf.kernel_launches++;
+  }
+  CUDA_TRY(h, cudaEventRecord(h->ev1, s));
+  unsigned long long cnt[4] = {0, 0, 0, 0};
+  CUDA_TRY(h, cudaMemcpyAsync(first_hit, d_fh, (size_t)n_tests * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(h, cudaMemcpyAsync(first_bad, d_fb, (size_t)n_tests * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(h, cudaMemcpyAsync(cnt, h->counters_dev, sizeof(cnt), cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(h, cudaStreamSynchronize(s));
+  // the test stopped at the lower of the two; the other one is "none"
+  for (uint32_t t = 0; t < n_tests; t++) {
+    if (first_hit[t] < first_bad[t]) first_bad[t] = K;
+    else if (first_bad[t] < first_hit[t]) first_hit[t] = K;
+  }
+  float ms = 0;
+  CUDA_TRY(h, cudaEventElapsedTime(&ms, h->ev0, h->ev1));
+  h->perf.kernel_ms = ms;
+  h->perf.prefixes = cnt[3];
+  h->perf.deliveries = cnt[0];
+  h->perf.violations = cnt[1];
+  h->perf.deferred = (uint32_t)std::min<unsigned long long>(cnt[2], 0xFFFFFFFFull);
+  h->perf.h2d_bytes = stage.size();
+  h->perf.d2h_bytes = (size_t)n_tests * 8 + sizeof(cnt);
   return DEMI_OK;
 }
 

@@ -23,6 +23,7 @@ struct DDMinDriver {
   std::map<Mask, bool> memo;           // mask -> violation reproduced?
   uint32_t original_num_events = 0, total_inputs_pruned = 0, total_replays = 0;
   std::vector<uint32_t> iteration_sizes;
+  std::vector<uint32_t> iteration_keys;   // stats.total_replays when each iteration size was recorded (replay_count())
   uint32_t replays_executed = 0, batches = 0;
   int32_t error = DEMI_OK;
   bool malformed = false;
@@ -218,6 +219,8 @@ struct DDMinDriver {
   virtual int32_t evaluate_batch(const std::vector<Mask>& want, std::vector<char>& out) = 0;
   // the sequential walk consumed the result of test(m)
   virtual void consumed(const Mask&) {}
+  // MinimizationStats.total_replays as the oracle counts it (one per test here; RandomScheduler: one per execution)
+  virtual uint32_t replay_count() const { return total_replays; }
   virtual ~DDMinDriver() {}
 
   void evaluate(std::vector<Mask>& want) {
@@ -272,6 +275,7 @@ struct DDMinDriver {
       if (error != DEMI_OK) return dag;
       total_replays++;
       iteration_sizes.push_back(original_num_events - total_inputs_pruned);
+      iteration_keys.push_back(replay_count());
       if (violates) {
         total_inputs_pruned += dag_len - popcount(hv[k]);
         return ddmin2(hv[k], rem);

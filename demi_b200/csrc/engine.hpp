@@ -79,6 +79,7 @@ struct demi_handle {
   // ---- launch bookkeeping
   std::map<const void*, int> occupancy;          // kernel -> resident blocks per SM (asked once per handle)
   void* trace_rec = nullptr; size_t trace_rec_bytes = 0;   // demi_fuzz_trace's recording buffer
+  void* subseq_buf = nullptr; size_t subseq_buf_bytes = 0; // demi_fuzz_subseq_batch: per-test side tables + verdicts
 };
 void demi_replay_free(demi_handle* h);
 void demi_comm_free(demi_handle* h);

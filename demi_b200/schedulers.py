@@ -205,6 +205,36 @@ class Engine(object):
                                        mcs.ctypes.data, mw, iters.ctypes.data, cap_iterations, C.byref(out)))
         return mcs, iters[:min(out.n_iterations, cap_iterations)].copy(), out
 
+    def fuzz_subseq_batch(self, masks, max_executions, max_messages, interval, seed_base=0, looking_for=0):
+        """RandomScheduler.test(program_of(mask_t)) for every row of `masks` (uint64 [n_tests, mask_words] over the
+        program given to set_externals), K = max_executions executions each, in one batch.  Returns (first_hit,
+        first_bad): per test the first execution that ends on a matching violation / a capacity status, K if none."""
+        masks = np.ascontiguousarray(np.atleast_2d(masks), dtype=np.uint64)
+        n = len(masks)
+        hit, bad = np.empty(n, dtype=np.uint32), np.empty(n, dtype=np.uint32)
+        p = N.FuzzParams(seed_base, max_executions, max_messages, interval, looking_for or 0, 0)
+        self._check(N.lib().demi_fuzz_subseq_batch(self._h, C.byref(p), masks.ctypes.data if n else None, n,
+                                                   masks.shape[1], hit.ctypes.data, bad.ctypes.data))
+        return hit, bad
+
+    def random_ddmin(self, max_executions, max_messages, interval, seed_base=0, looking_for=0, conjoin_pairs=(),
+                     check_unmodified=False, cap_iterations=1 << 16):
+        """RunnerUtils.randomDDMin's DDMin over the program given to set_externals (demi_random_ddmin).  Returns
+        (mcs mask, iteration sizes, iteration keys, demi_ddmin_out, verify seed or None)."""
+        n_ext = len(self._ext) if self._ext is not None else 0
+        mw = max(1, (n_ext + 63) // 64)
+        mcs = np.zeros(mw, dtype=np.uint64)
+        sizes = np.zeros(cap_iterations, dtype=np.uint32)
+        keys = np.zeros(cap_iterations, dtype=np.uint32)
+        pairs = np.ascontiguousarray(np.array(list(conjoin_pairs), dtype=np.uint32).reshape(-1, 2))
+        p = N.FuzzParams(seed_base, max_executions, max_messages, interval, looking_for or 0, 0)
+        out, vs = N.DDMinOut(), C.c_int64()
+        self._check(N.lib().demi_random_ddmin(self._h, C.byref(p), pairs.ctypes.data if len(pairs) else None, len(pairs),
+                                              1 if check_unmodified else 0, mcs.ctypes.data, mw, sizes.ctypes.data,
+                                              keys.ctypes.data, cap_iterations, C.byref(out), C.byref(vs)))
+        k = min(out.n_iterations, cap_iterations)
+        return mcs, sizes[:k].copy(), keys[:k].copy(), out, (vs.value if vs.value >= 0 else None)
+
     # ---- state-hash dedup + compaction (K5 / K4)
     def dedup_compact(self, results, mode=0):
         results = np.ascontiguousarray(results, dtype=N.RESULT_DTYPE)
@@ -414,6 +444,27 @@ def events_of(externals, mask):
     return [e for i, e in enumerate(externals) if (int(mask[i // 64]) >> (i % 64)) & 1]
 
 
+def program_of(externals, mask):
+    """The program a RandomScheduler test of subsequence `mask` runs (include/demi_b200.h, demi_fuzz_subseq_batch):
+    the selected externals in order, except that a selected WaitQuiescence right after another selected
+    WaitQuiescence is left out.  `externals`: packed records (EXT_DTYPE) or a list of events; the result has the
+    same form."""
+    packed = isinstance(externals, np.ndarray)
+    kinds = externals["kind"] if packed else pack_externals(list(externals))["kind"]
+    keep, prev_wq = [], False
+    for i in range(len(kinds)):
+        if not (int(mask[i // 64]) >> (i % 64)) & 1:
+            continue
+        wq = int(kinds[i]) == N.EXT_WAIT_QUIESCENCE
+        if wq and prev_wq:
+            continue
+        prev_wq = wq
+        keep.append(i)
+    if not keep:
+        raise ValueError("program_of: the mask selects no external")
+    return externals[np.array(keep, dtype=np.int64)] if packed else [externals[i] for i in keep]
+
+
 from .minimization_stats import MinimizationStats  # noqa: E402  (minification/Minimizer.scala:30-237)
 
 
@@ -475,32 +526,106 @@ class ReplayScheduler(STSScheduler):
 
 class DDMin(object):
     """DDMin(oracle, checkUnmodifed) — minification/DeltaDebugging.scala:7-109, with an
-    STSScheduler as the TestOracle (RunnerUtils.stsSchedDDMin, RunnerUtils.scala:642-707)."""
+    STSScheduler as the TestOracle (RunnerUtils.stsSchedDDMin, RunnerUtils.scala:642-707), or with a
+    RandomScheduler (RunnerUtils.randomDDMin, RunnerUtils.scala:601-623).  With a RandomScheduler, minimize()
+    takes the externals to minimize (the dag, WaitQuiescence included) and runs demi_random_ddmin on the
+    scheduler's engine; the engine's program is left as it was."""
 
     def __init__(self, oracle, checkUnmodifed=False, stats=None):
         self.oracle = oracle
         self.checkUnmodifed = checkUnmodifed
         self._stats = stats or MinimizationStats()
         self.last = None
+        self.verify_seed = None
+        self._conjoined = []
+
+    def _random(self):
+        return isinstance(self.oracle, RandomScheduler)
 
     def conjoinAtoms(self, e1, e2):
         """UnmodifiedEventDag.conjoinAtoms (minification/Util.scala:167-178) on the dag DDMin minimizes."""
+        if self._random():
+            self._conjoined.append((e1, e2))       # resolved against the externals given to minimize()
+            return
         ext = self.oracle.original_externals
         for e in (e1, e2):
             if e not in ext:
                 raise ValueError("No such external event:%r" % (e,))
         self.oracle.engine.conjoin_atoms(ext.index(e1), ext.index(e2))
 
-    def minimize(self, violation_fingerprint):
-        """Returns the MCS as a list of ExternalEvents (WaitQuiescence dropped, RunnerUtils.scala:678-684)."""
+    def minimize(self, violation_fingerprint, externals=None):
+        """STSScheduler: minimize(violation) returns the MCS as a list of ExternalEvents (WaitQuiescence dropped,
+        RunnerUtils.scala:678-684).  RandomScheduler: minimize(violation, externals) returns the MCS of `externals`."""
+        if self._random():
+            return self._minimize_random(violation_fingerprint, externals)
         mcs, iters, out = self.oracle.engine.ddmin(violation_fingerprint, self.oracle.flags, self.checkUnmodifed)
         self._stats.record_series(iters)
         self._stats.total_replays = out.total_replays
         self.last = out
         return events_of(self.oracle.original_externals, mcs)
 
+    def _minimize_random(self, violation_fingerprint, externals):
+        if externals is None:
+            raise ValueError("DDMin with a RandomScheduler: minimize(violation, externals)")
+        if self.oracle.test_invariant is None:
+            raise ValueError("Must invoke setInvariant before test()")
+        ext = list(externals)
+        ids = [e._id for e in ext]
+        pairs = []
+        for e1, e2 in self._conjoined:
+            for e in (e1, e2):
+                if e._id not in ids:
+                    raise ValueError("No such external event:%r" % (e,))
+            pairs.append((ids.index(e1._id), ids.index(e2._id)))
+        eng = self.oracle.engine
+        saved = eng._ext
+        eng.set_externals(ext)
+        try:
+            mcs, sizes, keys, out, vseed = eng.random_ddmin(
+                self.oracle.max_executions, self.oracle.maxMessages, self.oracle.invariant_check_interval,
+                self.oracle.seed, violation_fingerprint, pairs, self.checkUnmodifed)
+        finally:
+            if saved is not None:
+                eng.set_externals(saved)
+        inner = self._stats.inner()
+        for k, v in zip(keys, sizes):                 # MinimizationStats.iterationSize (Minimizer.scala:183-185)
+            inner.iterationSize[int(k)] = int(v)
+            inner.iteration_size_log.append(int(v))
+        self._stats.total_replays = out.total_replays
+        self.last, self.verify_seed = out, vseed
+        self.mcs_mask = mcs
+        return events_of(ext, mcs)
+
     def verify_mcs(self, mcs, violation_fingerprint):
         return self.oracle.test(mcs, violation_fingerprint)
+
+
+def random_ddmin(experiment, schedulerConfig, max_executions=1, seed=0, stats=None, interval=0):
+    """RunnerUtils.randomDDMin (RunnerUtils.scala:601-623) over `experiment` (experiment.load_experiment output):
+    DDMin of its original externals with RandomScheduler(schedulerConfig, max_executions, interval, FullyRandom(seed + i)
+    for execution i) as the TestOracle, setMaxMessages(len(trace)) (:608), checkUnmodifed = false (:610).
+    Returns (mcs events, stats, EventTrace | None, violation).  The EventTrace is the recorded execution of the
+    MCS's violating verification run (demi_fuzz_trace on program_of(mcs), recorded on an Engine of its own), or the
+    experiment's trace when nothing was removed."""
+    from .events import unpack_externals
+    ext = unpack_externals(experiment["externals"])
+    trace = experiment["events"]
+    violation = int(experiment["meta"]["violation"])
+    sched = RandomScheduler(schedulerConfig, max_executions, interval, seed)
+    sched.setMaxMessages(len(trace))
+    ddmin = DDMin(sched, checkUnmodifed=False, stats=stats)
+    mcs = ddmin.minimize(violation, ext)
+    if len(mcs) < len(ext):
+        validated = None
+        if ddmin.verify_seed is not None:
+            rec = Engine(schedulerConfig)
+            try:
+                rec.set_externals(program_of(ext, ddmin.mcs_mask))
+                validated = rec.fuzz_trace(ddmin.verify_seed, sched.maxMessages, interval, violation)[0]
+            finally:
+                rec.close()
+        return mcs, ddmin._stats, validated, violation
+    return mcs, ddmin._stats, trace, violation
 
 
 class ProvenanceTracker:

@@ -314,6 +314,42 @@ int32_t demi_ddmin(demi_handle* h, uint32_t looking_for, uint32_t flags, int32_t
                    uint64_t* mcs_mask, uint32_t mask_words,
                    uint32_t* iteration_sizes, uint32_t cap_iterations, demi_ddmin_out* out);
 
+/* ------------------------------------------------- DDMin with RandomScheduler */
+/* program_of(mask): the externals of the program given to demi_set_externals whose bit is set (bit j selects
+ * external j), in their order, except that a selected WaitQuiescence whose previous selected external is also a
+ * WaitQuiescence is left out (DDMin can make two of them adjacent; demi_set_externals rejects that, and the second
+ * would wait for a quiescence that already holds).  An all-zero mask, or a bit at or beyond n_ext, is
+ * DEMI_ERR_INVALID.
+ *
+ * Test t = RandomScheduler(cfg, max_executions = K = p->n_prefixes, p->invariant_check_interval,
+ * FullyRandom(p->seed_base + i) for execution i).test(program_of(mask_t), p->looking_for), run the reference's way:
+ * executions i = 0, 1, ... until the first that ends on a matching violation (a hit) or on a capacity status
+ * (DEMI_PS_*; the capacities are those of program_of(mask_t) with its own number of Sends, demi_limits.h).
+ * first_hit[t] = that execution if it was a hit, else K; first_bad[t] = that execution if it ended on a status,
+ * else K.  At most one of the two is below K.  The same numbers come from demi_set_externals(program_of(mask_t)) +
+ * demi_fuzz_batch(seed_base, K): the first record with a nonzero violation or status.  Every test runs in one
+ * batch: item i*n_tests + t is execution i of test t, and items of a test that already stopped are skipped; no
+ * per-execution record is written.  demi_stats: prefixes = executions actually run, deferred as for fuzz.  The
+ * handle's program is not changed. */
+int32_t demi_fuzz_subseq_batch(demi_handle* h, const demi_fuzz_params* p, const uint64_t* masks, uint32_t n_tests,
+                               uint32_t mask_words, uint32_t* first_hit, uint32_t* first_bad);
+/* RunnerUtils.randomDDMin (RunnerUtils.scala:601-623): DDMin (DeltaDebugging.scala:27-109) over the whole program
+ * given to demi_set_externals, WaitQuiescence included, with the tests above as the TestOracle.  Kill/Start,
+ * Partition/UnPartition and the conjoin_pairs (n_pairs (e1, e2) index pairs, UnmodifiedEventDag.conjoinAtoms) are
+ * atoms.  Decisions, MCS and iteration_sizes are the sequential ones; tests are evaluated speculatively in batches.
+ * out->total_replays = executions the sequential run issues (RandomScheduler counts one per execution it runs,
+ * RandomScheduler.scala:248-253: first_hit + 1, or K without a hit); iteration_keys[k] = total_replays when
+ * iteration_sizes[k] was recorded (MinimizationStats.iterationSize, Minimizer.scala:183-185).  check_unmodified
+ * tests the whole program first and is not counted.  A test that ends on a capacity status, when the sequential
+ * walk consumes it, is DEMI_ERR_CAPACITY.  out->verified / *verify_seed: verify_mcs, one more test of the MCS, and
+ * the seed of its violating execution (-1 if none), for demi_fuzz_trace on program_of(mcs).  out->replays_executed
+ * = tests evaluated (speculation included), out->batches = demi_fuzz_subseq_batch calls.  The handle's program is
+ * not changed. */
+int32_t demi_random_ddmin(demi_handle* h, const demi_fuzz_params* p, const uint32_t* conjoin_pairs, uint32_t n_pairs,
+                          int32_t check_unmodified, uint64_t* mcs_mask, uint32_t mask_words,
+                          uint32_t* iteration_sizes, uint32_t* iteration_keys, uint32_t cap_iterations,
+                          demi_ddmin_out* out, int64_t* verify_seed);
+
 /* --------------------------------------------------------------------- DPOR */
 /* DPORwHeuristics(schedulerConfig, backtrackHeuristic = DefaultBacktrackOrdering,
  * depth_bound, stopIfViolationFound, trackHistory = true) driven like

@@ -221,6 +221,11 @@ class RandomScheduler {
     if (!r) return std::nullopt;
     return r->first;
   }
+  // the parameters of one test (DDMin with this scheduler as its oracle runs many at once)
+  demi_fuzz_params params(ViolationFingerprint lookingFor) const {
+    return demi_fuzz_params{seed, max_executions, maxMessages, invariant_check_interval, lookingFor, 0};
+  }
+  bool invariant_set() const { return have_invariant; }
   std::shared_ptr<Engine> engine;
   std::vector<demi_fuzz_result> results;
   std::vector<uint16_t> depGraph;      // depTracker.getGraph of the violating execution, as parent pointers
@@ -288,24 +293,57 @@ class ReplayScheduler : public STSScheduler {
 class DDMin {
  public:
   DDMin(STSScheduler& oracle, bool checkUnmodifed = false, MinimizationStats* stats = nullptr)
-      : oracle(oracle), checkUnmodifed(checkUnmodifed), _stats(stats ? stats : &own) {}
+      : _stats(stats ? stats : &own), oracle(&oracle), checkUnmodifed(checkUnmodifed) {}
+  // RunnerUtils.randomDDMin (RunnerUtils.scala:601-623): RandomScheduler as the TestOracle (demi_random_ddmin)
+  DDMin(RandomScheduler& oracle, bool checkUnmodifed = false, MinimizationStats* stats = nullptr)
+      : _stats(stats ? stats : &own), random(&oracle), checkUnmodifed(checkUnmodifed) {}
   // the MCS (WaitQuiescence dropped, RunnerUtils.scala:678-684); throws std::invalid_argument
   // ("Unmodified trace does not trigger violation") like DeltaDebugging.scala:41-47
   ExternalEvents minimize(ViolationFingerprint fp) {
-    std::vector<uint64_t> mcs(oracle.mask_words(), 0);
+    if (!oracle) throw std::invalid_argument("DDMin with a RandomScheduler: minimize(fp, externals)");
+    std::vector<uint64_t> mcs(oracle->mask_words(), 0);
     std::vector<uint32_t> iters(1 << 16);
-    oracle.engine->check(demi_ddmin(oracle.engine->handle(), fp, oracle.flags, checkUnmodifed ? 1 : 0, mcs.data(),
-                                    oracle.mask_words(), iters.data(), (uint32_t)iters.size(), &last));
+    oracle->engine->check(demi_ddmin(oracle->engine->handle(), fp, oracle->flags, checkUnmodifed ? 1 : 0, mcs.data(),
+                                     oracle->mask_words(), iters.data(), (uint32_t)iters.size(), &last));
     _stats->iteration_size.clear();
     _stats->record_series(iters.data(), last.n_iterations, false);
     _stats->total_replays_ref() = last.total_replays;
-    return events_of(oracle.original_externals, mcs);
+    return events_of(oracle->original_externals, mcs);
   }
-  std::optional<EventTrace> verify_mcs(const ExternalEvents& mcs, ViolationFingerprint fp) { return oracle.test(mcs, fp); }
+  // RandomScheduler oracle: the MCS of `externals` (WaitQuiescence included, RunnerUtils.scala:607-611).  The
+  // scheduler's engine runs `externals` for the call and gets its previous program back (`restore`) afterwards.
+  ExternalEvents minimize(ViolationFingerprint fp, const ExternalEvents& externals, const ExternalEvents& restore = {}) {
+    if (!random) return minimize(fp);
+    if (!random->invariant_set()) throw std::invalid_argument("Must invoke setInvariant before test()");
+    Engine& e = *random->engine;
+    const uint32_t mw = (uint32_t)((externals.size() + 63) / 64 ? (externals.size() + 63) / 64 : 1);
+    std::vector<uint64_t> mcs(mw, 0);
+    std::vector<uint32_t> sizes(1 << 16), keys(1 << 16);
+    const demi_fuzz_params p = random->params(fp);
+    e.check(demi_set_externals(e.handle(), externals.data(), (uint32_t)externals.size()));
+    const int32_t rc = demi_random_ddmin(e.handle(), &p, conjoined.data(), (uint32_t)(conjoined.size() / 2), checkUnmodifed ? 1 : 0,
+                                         mcs.data(), mw, sizes.data(), keys.data(), (uint32_t)sizes.size(), &last, &verify_seed);
+    if (!restore.empty()) demi_set_externals(e.handle(), restore.data(), (uint32_t)restore.size());
+    e.check(rc);
+    _stats->iteration_size.clear();
+    for (uint32_t i = 0; i < last.n_iterations && i < sizes.size(); i++) {    // MinimizationStats.iterationSize (Minimizer.scala:183-185)
+      _stats->inner().iterationSize[keys[i]] = sizes[i];
+      _stats->iteration_size.push_back(sizes[i]);
+    }
+    _stats->total_replays_ref() = last.total_replays;
+    return events_of(externals, mcs);
+  }
+  // UnmodifiedEventDag.conjoinAtoms for the RandomScheduler form: indices into the externals given to minimize()
+  void conjoinAtoms(uint32_t i1, uint32_t i2) { conjoined.push_back(i1); conjoined.push_back(i2); }
+  std::optional<EventTrace> verify_mcs(const ExternalEvents& mcs, ViolationFingerprint fp) {
+    return oracle ? oracle->test(mcs, fp) : random->test(mcs, fp);
+  }
   demi_ddmin_out last{};
+  int64_t verify_seed = -1;            // RandomScheduler oracle: seed of the MCS's violating verification execution
   MinimizationStats* _stats;
  private:
-  STSScheduler& oracle; bool checkUnmodifed; MinimizationStats own;
+  STSScheduler* oracle = nullptr; RandomScheduler* random = nullptr; bool checkUnmodifed; MinimizationStats own;
+  std::vector<uint32_t> conjoined;
 };
 
 struct LeftToRightOneAtATime {};       // RemovalStrategy (OneAtATimeRemoval.scala:131-137)
